@@ -353,6 +353,26 @@ def run_cfg5(args, torch, tdist, dist, lio, synth, rank, world, local, stream, f
     return out
 
 
+def step_outputs(leg, last, eskf):
+    """What a caller of the timed path receives from one step: the registered pose, the filter state and the pass summary.
+    `last` is (summary, frame_q, frame_t) on one GPU, the result dict of DistributedLio on several."""
+    if isinstance(last, dict):
+        fq, ft = last["frame_q"], last["frame_t"]
+        summary, trace = [last["success"], last["passes"], last["num_residuals_used"], last["converged"]], last["trace"]
+    else:
+        s, fq, ft = last
+        summary, trace = [s.success, s.passes_run, s.num_residuals_used, s.converged], s.trace
+    out = {f"{leg}_frame_q": fq, f"{leg}_frame_t": ft, f"{leg}_summary": summary, f"{leg}_trace": trace,
+           **{f"{leg}_{f}": getattr(eskf, f) for f in ("p", "q", "v", "ba", "bg", "g", "cov")}}
+    return out
+
+
+def dump_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -385,10 +405,14 @@ def main():
                                                         "on by default when --gpus > 1")
     ap.add_argument("--no-cfg5", action="store_true")
     ap.add_argument("--cfg5-steps", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (float64), "
+                                                           "so that two builds can be compared output for output")
     args = ap.parse_args()
     global N_PASSES
     N_PASSES = args.passes
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of the GPU path (--impl b200)")
         return run_reference(args)
 
     import torch
@@ -441,9 +465,10 @@ def main():
         if world > 1:
             out = D.updateIEKF(prm, sw.t_last)
             assert out["success"] and out["passes"] == N_PASSES
-        else:
-            summ, _, _ = L.updateIEKF(prm, sw.t_last)
-            assert summ.success and summ.passes_run == N_PASSES, (summ.success, summ.passes_run)
+            return out
+        summ, fq, ft = L.updateIEKF(prm, sw.t_last)
+        assert summ.success and summ.passes_run == N_PASSES, (summ.success, summ.passes_run)
+        return summ, fq, ft
 
     # e2e leg: the host buffers a caller would hand over, in pinned memory (the contract's "from pinned host memory")
     pin_world = torch.empty((args.points, 3), dtype=torch.float64).pin_memory()
@@ -457,9 +482,10 @@ def main():
         if world > 1:
             out = D.optimize(raw_h, prm, sw.t_last, world_out=world_out)   # srl_optimize_host_dist: all in C, pinned buffers
             assert out["success"] and out["passes"] == N_PASSES
-        else:
-            summ, _, _, w = L.optimize(raw_h, prm, sw.t_last, want_world=True, world_out=world_out)
-            assert summ.success and summ.passes_run == N_PASSES
+            return out
+        summ, fq, ft, w = L.optimize(raw_h, prm, sw.t_last, want_world=True, world_out=world_out)
+        assert summ.success and summ.passes_run == N_PASSES
+        return summ, fq, ft
 
     def barrier():
         if world > 1:
@@ -475,6 +501,7 @@ def main():
         L.ctx.pass_time(reset=True)
         launches0 = L.ctx.kernel_launches
         barrier()
+        last = None
         for i in range(n_steps):
             sw = prepare(args.warmup + i) if with_prepare else sweeps[(args.warmup + i) % len(sweeps)]
             if not args.no_flush:
@@ -482,27 +509,30 @@ def main():
             if world > 1:
                 tdist.barrier()
             ev[i][0].record()
-            step_fn(sw)
+            last = step_fn(sw)
             ev[i][1].record()
         barrier()
         ms = np.array([a.elapsed_time(b) for a, b in ev])
         k1_ms, k1_n = L.ctx.pass_time(reset=True)
-        return ms, k1_ms, k1_n, L.ctx.kernel_launches - launches0
+        return ms, k1_ms, k1_n, L.ctx.kernel_launches - launches0, last
 
     clocks = ClockSampler(local)
     clocks.start()
-    ms_res, _, _, launches = timed(step_resident, True)
+    ms_res, _, _, launches, last_res = timed(step_resident, True)
+    outputs = step_outputs("resident", last_res, L.eskf_pro) if args.dump_outputs else None
     step_cycles = L.ctx.counter("iekf_step_cycles_avg")
     loop_on_device = bool(L.ctx.counter("device_loop_active"))
     order_impl = {1: "single-launch cluster radix sort (k_sweep_order_cluster), verified against the CUB order at first use",
                   0: "CUB radix sort", -1: "cluster radix sort, still in its first verified uses"}.get(L.ctx.counter("cluster_order_active"), "?")
     stage_cycles = [L.ctx.counter(f"iekf_stage_{i}") for i in range(8)]
-    ms_e2e, _, _, _ = timed(step_e2e, False)
+    ms_e2e, _, _, _, last_e2e = timed(step_e2e, False)
+    if outputs is not None:
+        outputs.update(step_outputs("e2e", last_e2e, L.eskf_pro), e2e_world=world_out.copy())
     # roofline leg: the same resident steps again with CUDA events around every pass's launches on the launching stream
     # (the events sit between the kernels, so this leg runs without programmatic dependent launch; its step time is
     # reported next to the main one)
     L.ctx.set_timing(True)
-    ms_tim, k1_ms, k1_n, _ = timed(step_resident, True, n_steps=min(args.steps, 40))
+    ms_tim, k1_ms, k1_n, _, _ = timed(step_resident, True, n_steps=min(args.steps, 40))
     L.ctx.set_timing(False)
     clk = clocks.stop()   # sampled over the three timed regions
 
@@ -684,6 +714,8 @@ def main():
             line["cfg5"] = cfg5
         if pose_check is not None:
             line["pose_check"] = pose_check
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     if D is not None:
         D.close()

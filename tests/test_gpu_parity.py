@@ -14,6 +14,9 @@ from sr_livo_b200 import synth
 pytestmark = pytest.mark.gpu
 BIG = 2 ** 31 - 1
 REL = 1e-5
+# the cases of the comparisons with the compiled reference (its outputs: tests/test_reference_pin.py, test_small_world_*)
+SMALL_WORLD_PASS = [dict(max_num_residuals=BIG), dict(max_num_residuals=BIG, frame_id=5), dict(max_num_residuals=600)]
+SMALL_WORLD_UPDATE = [dict(max_num_residuals=BIG), dict(max_num_residuals=600)]
 
 
 @pytest.fixture(scope="module")
@@ -1106,53 +1109,59 @@ def test_fused_peer_memory_exchange_ranks(tmp_path, world):
 
 
 # ---- the CUDA path against the REFERENCE'S OWN CODE (oracle/_ref/libsrl_reference.so, compiled where it lies) ------
+# Its outputs on this scene are recorded by tests/test_reference_pin.py (test_small_world_*) in tests/golden/reference_pin.npz.
 def _reference_or_skip():
     from oracle import reference_py as Rf
     if not Rf.available():
-        pytest.skip("oracle/_ref/libsrl_reference.so did not travel to this box")
+        pytest.skip("oracle/_ref/libsrl_reference.so was not built: the reference sources are absent")
     return Rf
 
 
-@pytest.mark.parametrize("kw", [dict(max_num_residuals=BIG), dict(max_num_residuals=BIG, frame_id=5), dict(max_num_residuals=600)])
-def test_gpu_pass_equals_the_compiled_reference(L, small_world, kw):
-    """One ESIKF pass on the GPU vs lioOptimization::buildPlaneResiduals of the reference's own src/optimize.cpp (no oracle in
-    between): transformed keypoints bit for bit, the same keypoints accepted in the same order, rows within 1e-5."""
+@pytest.fixture(scope="module")
+def ref_pin():
+    from refstore import Store
+    return Store("reference_pin.npz")
+
+
+@pytest.mark.parametrize("kw", SMALL_WORLD_PASS)
+def test_gpu_pass_equals_the_compiled_reference(L, small_world, ref_pin, kw):
+    """One ESIKF pass on the GPU vs lioOptimization::buildPlaneResiduals of the reference's own src/optimize.cpp: transformed
+    keypoints bit for bit, the same keypoints accepted in the same order, rows within 1e-5.  The reference's rows are stored as a
+    digest: the oracle's rows, which have that digest, stand for them."""
+    from refstore import digest, from_near
     from sr_livo_b200 import lio
-    Rf = _reference_or_skip()
+    r = ref_pin.get(f"small_world.pass{SMALL_WORLD_PASS.index(kw)}")
     om, sw = _load_world(L, small_world)
-    ref = Rf.Reference()
-    ref.load(*om.snapshot())
+    o = om.build_plane_residuals(sw.raw_xyz, sw.q_init, sw.t_init, sw.t_last, O.r3live_params(**kw), debug=True)
+    rows = o.plane[o.status == 2][:, :15]
+    assert r["rows"] == digest(rows)
+    ref_world = from_near(r, "world_all", o.world_xyz)
     L.setKeypoints(sw.raw_xyz)
     g = L.buildPlaneResiduals(lio.r3live_params(**kw), sw.q_init, sw.t_init, sw.t_last, debug=True)
-    r = ref.build_plane_residuals(sw.raw_xyz, sw.q_init, sw.t_init, sw.t_last, O.r3live_params(**kw))
     assert not r["threw"] and r["success"] == g.success and r["num_residuals_used"] == g.num_residuals
     visited = g.status >= 0
-    assert np.array_equal(g.world_xyz[visited], r["world_xyz"][visited])
+    assert np.array_equal(g.world_xyz[visited], ref_world[visited])
     got = g.plane[g.status == 2][:, :15]
-    assert got.shape == r["rows"].shape
-    scale = np.maximum(np.abs(r["rows"]).max(axis=0), 1e-12)
-    assert np.all(np.abs(got - r["rows"]) <= REL * scale)
+    assert got.shape == rows.shape
+    scale = np.maximum(np.abs(rows).max(axis=0), 1e-12)
+    assert np.all(np.abs(got - rows) <= REL * scale)
     assert abs(g.loss_sum - r["loss_sum"]) <= REL * r["loss_sum"]
 
 
-def test_gpu_update_equals_the_compiled_reference(L, small_world):
+def test_gpu_update_equals_the_compiled_reference(L, small_world, ref_pin):
     """updateIEKF on the GPU (device-resident loop) vs the reference's own updateIEKF + eskfEstimator::observe: state 1e-5."""
     from sr_livo_b200 import lio
-    Rf = _reference_or_skip()
     om, sw = _load_world(L, small_world)
-    ref = Rf.Reference()
-    ref.load(*om.snapshot())
     P = synth.prior_covariance()
-    for kw in (dict(max_num_residuals=BIG), dict(max_num_residuals=600)):
+    for case, kw in enumerate(SMALL_WORLD_UPDATE):
+        r = ref_pin.get(f"small_world.update{case}")
         L.setKeypoints(sw.raw_xyz)
         L.eskf_pro = lio.EskfEstimator(p=sw.t_init.copy(), q=sw.q_init.copy(), v=np.array([0.3, 0.0, 0.0]), cov=P.copy())
         summ, fq, ft = L.updateIEKF(lio.r3live_params(**kw), sw.t_last)
-        r = ref.update_iekf(sw.raw_xyz, O.Eskf(p=sw.t_init.copy(), q=sw.q_init.copy(), v=np.array([0.3, 0.0, 0.0]), cov=P.copy()), sw.t_last,
-                            O.r3live_params(**kw))
         assert not r["threw"] and summ.success == r["success"] and summ.num_residuals_used == r["num_residuals_used"]
         for f in ("p", "q", "v", "ba", "bg", "g"):
-            assert np.allclose(getattr(L.eskf_pro, f), getattr(r["eskf"], f), rtol=REL, atol=1e-9), f
-        assert np.allclose(L.eskf_pro.cov, r["eskf"].cov, rtol=1e-4, atol=1e-12)
+            assert np.allclose(getattr(L.eskf_pro, f), r[f], rtol=REL, atol=1e-9), f
+        assert np.allclose(L.eskf_pro.cov, r["cov"], rtol=1e-4, atol=1e-12)
         assert np.allclose(fq, r["frame_q"], atol=1e-9) and np.allclose(ft, r["frame_t"], atol=1e-9)
 
 
@@ -1163,7 +1172,7 @@ def test_reference_runs_on_the_gpu_backend(small_world):
     transformPoint) then registers a sweep through its own call sites on the GPU; the result equals the unpatched reference's."""
     Rf = _reference_or_skip()
     if not Rf.available(gpu=True):
-        pytest.skip("oracle/_ref/libsrl_reference_gpu.so did not travel to this box")
+        pytest.skip("oracle/_ref/libsrl_reference_gpu.so was not built: the reference sources are absent")
     pts, sw = small_world["pts"], small_world["sweep"]
     ref, rg = Rf.Reference(), Rf.Reference(gpu=True)
     assert ref.add_points_to_map(pts) > 0                       # the reference's own insertion into its host voxelHashMap

@@ -11,10 +11,20 @@ import numpy as np
 import pytest
 
 from oracle import oracle_py as O
+from oracle import reference_py as Rf
+from refstore import Store, eskf_fields
 from sr_livo_b200 import capi, dist, lio, synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIG = 2 ** 31 - 1
+
+
+@pytest.fixture(scope="module")
+def ref_out():
+    """outputs of the reference's own code (tests/refstore.py), stored in tests/golden/reference_host.npz"""
+    store = Store("reference_host.npz")
+    yield store
+    store.save()
 
 
 def test_library_exports_every_symbol_the_header_declares():
@@ -123,23 +133,24 @@ def test_iekf_host_algebra_matches_oracle(small_world, frame_id, thr_t):
 
 
 @pytest.mark.parametrize("kw", [dict(max_num_residuals=BIG), dict(max_num_residuals=BIG, threshold_translation_norm=0.0), dict(max_num_residuals=600)])
-def test_iekf_host_algebra_matches_the_compiled_reference(small_world, kw):
+def test_iekf_host_algebra_matches_the_compiled_reference(ref_out, small_world, kw):
     """The product's host ESIKF algebra (srl_iekf_begin / srl_iekf_step in libsrlivo_b200.so, driven here by oracle passes so that
     it runs without a GPU) against lioOptimization::updateIEKF of the reference's own src/optimize.cpp (oracle/_ref/libsrl_reference.so)."""
-    from oracle import reference_py as Rf
-    if not Rf.available():
-        pytest.skip("oracle/_ref/libsrl_reference.so not built")
     om, sw = small_world["omap"], small_world["sweep"]
     oprm, prm = O.r3live_params(**kw), capi.r3live_params(**kw)
     P = synth.prior_covariance()
-    ref = Rf.Reference()
-    ref.load(*om.snapshot())
-    r = ref.update_iekf(sw.raw_xyz, O.Eskf(p=sw.t_init.copy(), q=sw.q_init.copy(), cov=P.copy()), sw.t_last, oprm)
+
+    def rec():
+        ref = Rf.Reference()
+        ref.load(*om.snapshot())
+        res = ref.update_iekf(sw.raw_xyz, O.Eskf(p=sw.t_init.copy(), q=sw.q_init.copy(), cov=P.copy()), sw.t_last, oprm)
+        return dict(success=res["success"], threw=res["threw"], frame_q=res["frame_q"], frame_t=res["frame_t"], **eskf_fields(res["eskf"]))
+    r = ref_out("iekf." + "_".join(f"{k}{v}" for k, v in sorted(kw.items())), rec)
     est, trace, done = _run_product_host_loop(om, sw, oprm, prm, P)
     assert r["success"] and not r["threw"]
     for f in ("p", "q", "v", "ba", "bg", "g"):
-        assert np.allclose(getattr(est, f), getattr(r["eskf"], f), rtol=1e-9, atol=1e-11), f
-    assert np.allclose(est.cov, r["eskf"].cov, rtol=1e-6, atol=1e-11)
+        assert np.allclose(getattr(est, f), r[f], rtol=1e-9, atol=1e-11), f
+    assert np.allclose(est.cov, r["cov"], rtol=1e-6, atol=1e-11)
     assert np.allclose(trace[-1][17:20], r["frame_t"], rtol=0, atol=1e-11) and np.allclose(trace[-1][20:24], r["frame_q"], rtol=0, atol=1e-11)
 
 
@@ -157,31 +168,38 @@ def test_host_plane_fit_matches_numpy():
         assert abs(a2d.value - (np.sqrt(w[1]) - np.sqrt(abs(w[0]))) / np.sqrt(w[2])) < 1e-9
 
 
-def test_host_plane_fit_and_observe_match_the_compiled_reference():
+def test_host_plane_fit_and_observe_match_the_compiled_reference(ref_out):
     """srl_host_plane_fit (the plane fit of srl_math.cuh compiled for the host) and srl_eskf_observe against the reference's own
     computeNeighborhoodDistribution (src/optimize.cpp:316-353) and eskfEstimator::observe (src/eskfEstimator.cpp:219-230)."""
-    from oracle import reference_py as Rf
-    if not Rf.available():
-        pytest.skip("oracle/_ref/libsrl_reference.so not built")
-    ref = Rf.Reference()
     rng = np.random.default_rng(19)
+    sets = []
     for trial in range(200):
         P = rng.normal(size=(20, 3)) * np.array([0.5, 0.4, 0.01 * (1 + trial % 5)])
-        P = (P @ np.linalg.qr(rng.normal(size=(3, 3)))[0].T + rng.normal(size=3) * 30).astype(np.float32).astype(np.float64)
+        sets.append((P @ np.linalg.qr(rng.normal(size=(3, 3)))[0].T + rng.normal(size=3) * 30).astype(np.float32).astype(np.float64))
+
+    def rec():
+        ref = Rf.Reference()
+        out = [ref.neighborhood(P) for P in sets]
+        return dict(rc=np.array([rc for rc, _ in out]), normal=np.stack([nh["normal"] for _, nh in out]), a2D=np.array([nh["a2D"] for _, nh in out]))
+    r = ref_out("neighborhood", rec)
+    for trial, P in enumerate(sets):
         n = np.zeros(3); a2d = C.c_double(0); ev = np.zeros(3)
         assert capi.lib().srl_host_plane_fit(capi.ptr(P), 20, capi.ptr(n), C.byref(a2d), capi.ptr(ev)) == 0
-        rc, nh = ref.neighborhood(P)
-        assert rc == 0
-        assert abs(abs(n @ nh["normal"]) - 1) < 1e-9 and abs(a2d.value - nh["a2D"]) <= 1e-9 * max(1.0, abs(nh["a2D"]))
+        assert r["rc"][trial] == 0
+        a2d_ref = r["a2D"][trial]
+        assert abs(abs(n @ r["normal"][trial]) - 1) < 1e-9 and abs(a2d.value - a2d_ref) <= 1e-9 * max(1.0, abs(a2d_ref))
+    cases = []
     for trial in range(30):
         scale = [0.05, 1e-6, 0.5][trial % 3]
         kw = dict(p=rng.normal(size=3), q=synth.quat_from_rotvec(rng.normal(size=3)), v=rng.normal(size=3), ba=rng.normal(size=3) * 0.01,
                   bg=rng.normal(size=3) * 0.01, g=np.array([0.3, -0.2, 9.7]) + rng.normal(size=3) * 0.1)
-        dx = rng.normal(size=17) * scale
+        cases.append((kw, rng.normal(size=17) * scale))
+    names = ("p", "q", "v", "ba", "bg", "g")
+    r = ref_out("observe", lambda: {f: np.stack([getattr(Rf.eskf_observe(O.Eskf(**kw), dx), f) for kw, dx in cases]) for f in names})
+    for trial, (kw, dx) in enumerate(cases):
         a = lio.EskfEstimator(**kw).observe(dx)
-        b = Rf.eskf_observe(O.Eskf(**kw), dx)
-        for f in ("p", "q", "v", "ba", "bg", "g"):
-            assert np.allclose(getattr(a, f), getattr(b, f), rtol=0, atol=1e-14), f
+        for f in names:
+            assert np.allclose(getattr(a, f), r[f][trial], rtol=0, atol=1e-14), f
 
 
 def test_shard_ranges_cover_the_sweep_in_order():
